@@ -2,7 +2,7 @@
 """bench.py — scans/sec of the B200 scan-matching hot path, with the live roofline of its residual kernel, a parity block
 against the CPU oracle on the very scans that were timed, and the CPU oracle timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--batch B] [--dump-outputs DIR]
 
 One "step" = one batched Match of B synthetic scans per GPU against a static (replicated) map (SURVEY.md §8d/§8e).
 For N > 1 launch under torchrun (one rank per GPU): every rank matches its own B scans per step; the per-scan results
@@ -16,6 +16,10 @@ Timed legs (all inside this process, nothing under a profiler):
   roofline  same steps on a handle created with FLS_FLAG_PROFILE: CUDA events around every residual-kernel launch
   cpu_baseline / --impl reference: the CPU oracle (port of the reference algorithm, OpenMP; thread count chosen by a sweep)
   parity    GPU results of the scan pool vs the oracle's results for the same scans and guesses (N = 1, rank 0)
+
+--dump-outputs DIR writes what the last timed step of the `value` leg returned on rank 0 (the B scans of that step, all inputs
+seeded, so two builds run with the same arguments can be compared file by file): poses.npy (B,4,4), converged.npy,
+iterations.npy, n_source.npy, n_valid.npy and sum_residual.npy (B,), all float64.
 """
 from __future__ import annotations
 
@@ -263,6 +267,16 @@ def parity_block(gpu_res, orc_res):
             "against": "CPU oracle (port of the reference algorithm) on the same scans, guesses and map"}
 
 
+def dump_outputs(out_dir: str, oks, Ts, stats) -> None:
+    """Per-scan results of one step as float64 .npy files (see the module docstring)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"poses": np.asarray(Ts, np.float64), "converged": np.asarray(oks, np.float64)}
+    for name in ("iterations", "n_source", "n_valid", "sum_residual"):
+        arrays[name] = np.array([getattr(s, name) for s in stats], np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def secondary_kernels(device: int, peak: float, log, steps: int = 6):
     """Short measurements of the other §8 kernels (K2 NDT, K3 ICP, K4 features, K5 kd-tree LOAM) beside the headline: scans/s
     with the scan resident in HBM, live roofline of the residual kernel (CUDA events per launch), the CPU oracle on the same
@@ -433,7 +447,12 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the short K2/K3/K4/K5 side measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline + parity leg (profiling runs)")
     ap.add_argument("--batch", type=int, default=8, help="scans per GPU per step (one fls_match_batch call; BASELINE config 4 uses batches of 8)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's results: it needs --impl ours")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
@@ -480,6 +499,7 @@ def main():
     # device buffer and all-gathered over NCCL asynchronously; consumed two steps later (never inside the step)
     gather = parallel.AsyncResultGather(B, device=dev, depth=3)
     gathered_steps = [0]
+    last_step = {}  # host (e2e leg) or not (value leg) -> (converged, poses, stats) of the last timed step
 
     def flush_l2():
         flush_buf.zero_()
@@ -549,6 +569,7 @@ def main():
             d2h += sum(x.d2h_bytes for x in st)
             for j, T in zip(ids(warmup + i), Ts):
                 errs.append(synth.pose_error(T, truths[j]))
+        last_step[host] = (oks, Ts, st)
         # the collectives still in flight belong to the K timed steps: drain them inside the timed region
         e0.record()
         gather.drain()
@@ -602,6 +623,7 @@ def main():
                 acc[3] += sum(x.iterations for x in st)
                 for j, T in zip(ids(i), Ts):
                     acc[4].append(synth.pose_error(T, truths[j]))
+                last_step[host] = (oks, Ts, st)
 
         for i in range(warmup):
             begin(i)
@@ -731,6 +753,8 @@ def main():
     clocks = sampler.stop()
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *last_step[False])
         pos = float(np.median([e[0] for e in errs]))
         launch_us = 1e3 * k_ms / max(k_launch, 1)
         roof = {"bound": "hbm", "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak, "traffic": traffic,

@@ -1,14 +1,31 @@
 """Every `file:line` citation of the reference in the ABI header, the docs, the oracle and the CUDA sources must point at
-an existing file of the reference tree with at least that many lines.  Runs only where the read-only reference is mounted
-(the build container); skipped elsewhere (the GPU box has no /root/reference and nothing there needs it)."""
+an existing file of the reference tree with at least that many lines.  The reference tree is not part of this repository:
+the check runs against tests/golden/reference_line_counts.json, the path and line count of every file of that tree.
+Regenerate it from a checkout of the reference with  python tests/test_citations.py <reference-dir>"""
+import json
 import os
 import re
-
-import pytest
+import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+INDEX = os.path.join(ROOT, "tests", "golden", "reference_line_counts.json")
 PAT = re.compile(r"([A-Za-z0-9_/\.]+\.(?:h|cpp|yaml|md|txt)):(\d+)(?:-(\d+))?")
+
+
+def _n_lines(p):
+    with open(p, errors="ignore") as fh:
+        return sum(1 for _ in fh)
+
+
+def make_index(ref_dir):
+    """{path relative to the reference root: number of lines} of every file of the reference tree."""
+    out = {}
+    for d, dirs, fs in os.walk(ref_dir):
+        dirs[:] = sorted(x for x in dirs if x != ".git")
+        for f in sorted(fs):
+            p = os.path.join(d, f)
+            out[os.path.relpath(p, ref_dir)] = _n_lines(p)
+    return out
 
 
 def _sources():
@@ -18,18 +35,12 @@ def _sources():
     return out
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
 def test_reference_citations_resolve():
+    with open(INDEX) as fh:
+        index = json.load(fh)
     files = {}
-    for d, _, fs in os.walk(REF):
-        if "/.git" in d:
-            continue
-        for f in fs:
-            files.setdefault(f, []).append(os.path.join(d, f))
-
-    def n_lines(p):
-        with open(p, errors="ignore") as fh:
-            return sum(1 for _ in fh)
+    for rel, n in index.items():
+        files.setdefault(os.path.basename(rel), []).append(("/" + rel, n))
 
     checked, bad = 0, []
     for src in _sources():
@@ -41,10 +52,16 @@ def test_reference_citations_resolve():
             checked += 1
             cands = files.get(base, [])
             if "/" in path:
-                cands = [c for c in cands if c.endswith(path)] or cands
+                cands = [c for c in cands if c[0].endswith(path)] or cands
             if not cands:
                 bad.append((os.path.relpath(src, ROOT), m.group(0), "no such file in the reference"))
-            elif max(n_lines(c) for c in cands) < last:
+            elif max(n for _, n in cands) < last:
                 bad.append((os.path.relpath(src, ROOT), m.group(0), "file is shorter than the cited line"))
     assert checked > 150
     assert not bad, bad
+
+
+if __name__ == "__main__":
+    with open(INDEX, "w") as fh:
+        json.dump(make_index(sys.argv[1]), fh, indent=0, sort_keys=True)
+        fh.write("\n")
