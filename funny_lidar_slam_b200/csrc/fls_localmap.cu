@@ -77,21 +77,7 @@ int Handle::update_local_map(const double* T, int* updated, size_t* n_local) {
     if (updated) *updated = 1;
     if (m == 0) return FLS_OK;  // `local_map->empty()`: the caller gives up (:129-131); the matcher keeps its map
     // matcher_->AddCloudToLocalMap({*local_map}) (:135, :222) — the cloud is already on the device
-    switch (cfg.method) {
-        case FLS_P2PLANE_IVOX: {
-            if (cfg.localization_mode) ivox.clear();
-            else if (ivox.n_pts != 0) return FLS_ERR_UNSUPPORTED;
-            const int rc = ivox.append_and_build(stage2.p, m, cfg.ivox_capacity, stream);
-            launches += ivox.launches;
-            ivox.launches = 0;
-            if (cfg.localization_mode) set_fit_cloud(stage2.p, m);
-            return rc;
-        }
-        case FLS_NDT: return add_cloud_ndt(stage2.p, m);
-        case FLS_ICP_P2P: return add_cloud_icp(stage2.p, m);
-        case FLS_P2PLANE_KNN: return add_cloud_kd(stage2.p, m, nullptr, 0);
-        default: return FLS_ERR_UNSUPPORTED;  // LoamFull takes {planar, corner} maps
-    }
+    return add_cloud(stage2.p, m);
 }
 
 // ---- PCD --------------------------------------------------------------------------------------------------------------------

@@ -41,6 +41,33 @@ def _cloud(a):
     return a.ctypes.data_as(C.c_void_p), a.shape[0], a.shape[1] * 4, a
 
 
+def _pack(clouds):
+    """Host clouds -> (pointer array, count array, stride, arrays that must stay alive while the device may read them)."""
+    ptrs, ns, keep, stride = [], [], [], None
+    for c in clouds:
+        p, n, s, a = _cloud(c)
+        if stride is not None and s != stride:
+            raise ValueError("all clouds of one call must share a layout")
+        stride = s
+        ptrs.append(p)
+        ns.append(n)
+        keep.append(a)
+    return (C.c_void_p * len(ptrs))(*ptrs), (C.c_size_t * len(ns))(*ns), stride, keep
+
+
+def _pack_device(d_ptrs, ns):
+    return (C.c_void_p * len(d_ptrs))(*[int(p) for p in d_ptrs]), (C.c_size_t * len(ns))(*[int(n) for n in ns])
+
+
+def _colmajor(Ts):
+    """(B,4,4) poses -> a new float64 array holding each pose in Eigen's column-major memory order."""
+    return np.transpose(np.asarray(Ts, np.float64), (0, 2, 1)).copy()
+
+
+def _batch_out(B):
+    return (C.c_int * B)(), (FlsMatchStats * B)()
+
+
 class Registration:
     def __init__(self, cfg: FlsConfig):
         self.cfg = cfg
@@ -52,18 +79,8 @@ class Registration:
     def AddCloudToLocalMap(self, cloud_list) -> None:
         if isinstance(cloud_list, np.ndarray):
             cloud_list = [cloud_list]
-        ptrs, ns, keep, stride = [], [], [], None
-        for c in cloud_list:
-            p, n, s, a = _cloud(c)
-            if stride is not None and s != stride:
-                raise ValueError("all clouds of one call must share a layout")
-            stride = s
-            ptrs.append(p)
-            ns.append(n)
-            keep.append(a)
-        arr_p = (C.c_void_p * len(ptrs))(*ptrs)
-        arr_n = (C.c_size_t * len(ns))(*ns)
-        check(lib().fls_add_cloud(self._h, len(ptrs), arr_p, arr_n, stride), "fls_add_cloud")
+        arr_p, arr_n, stride, keep = _pack(cloud_list)
+        check(lib().fls_add_cloud(self._h, len(arr_p), arr_p, arr_n, stride), "fls_add_cloud")
 
     def Match(self, cluster: PointcloudCluster, T: np.ndarray) -> bool:
         """T: (4,4) float64, updated in place (also on failure, as upstream)."""
@@ -95,73 +112,41 @@ class Registration:
     def match_batch(self, scans, Ts):
         """scans: list of (n,4)/(n,8) host clouds; Ts: (B,4,4) float64 initial poses.  Returns (converged[B], T[B,4,4]);
         self.last_batch_stats holds the per-scan fls_match_stats (call-level timings on element 0)."""
-        B = len(scans)
-        ptrs, ns, keep, stride = [], [], [], None
-        for c in scans:
-            p, n, s, a = _cloud(c)
-            if stride is not None and s != stride:
-                raise ValueError("all scans of one batch must share a layout")
-            stride = s
-            ptrs.append(p)
-            ns.append(n)
-            keep.append(a)
-        Tc = np.ascontiguousarray(np.transpose(np.asarray(Ts, np.float64), (0, 2, 1))).copy()  # Eigen column-major per pose
-        conv = (C.c_int * B)()
-        st = (FlsMatchStats * B)()
-        arr_p = (C.c_void_p * B)(*ptrs)
-        arr_n = (C.c_size_t * B)(*ns)
-        check(lib().fls_match_batch(self._h, B, arr_p, arr_n, stride, Tc.ctypes.data_as(C.c_void_p), conv, st), "fls_match_batch")
-        self.last_batch_stats = list(st)
-        self.last_stats = st[0]
-        return np.array(conv[:], bool), np.transpose(Tc, (0, 2, 1)).copy()
+        arr_p, arr_n, stride, keep = _pack(scans)
+        Tc, (conv, st) = _colmajor(Ts), _batch_out(len(scans))
+        check(lib().fls_match_batch(self._h, len(scans), arr_p, arr_n, stride, Tc.ctypes.data_as(C.c_void_p), conv, st), "fls_match_batch")
+        return self._batch_result(Tc, conv, st)
 
     def match_batch_begin(self, scans, Ts) -> None:
         """First half of match_batch: enqueue copies + matching + read-back on the handle's stream, do not wait (the scans should sit
         in pinned host memory).  With two handles the copy of one batch overlaps the kernels of the other."""
-        B = len(scans)
-        ptrs, ns, keep, stride = [], [], [], None
-        for c in scans:
-            p, n, s, a = _cloud(c)
-            if stride is not None and s != stride:
-                raise ValueError("all scans of one batch must share a layout")
-            stride = s
-            ptrs.append(p)
-            ns.append(n)
-            keep.append(a)
-        Tc = np.ascontiguousarray(np.transpose(np.asarray(Ts, np.float64), (0, 2, 1))).copy()
-        arr_p = (C.c_void_p * B)(*ptrs)
-        arr_n = (C.c_size_t * B)(*ns)
-        self._pending = (keep, arr_p, arr_n, Tc, B)
-        check(lib().fls_match_batch_begin(self._h, B, arr_p, arr_n, stride, Tc.ctypes.data_as(C.c_void_p)), "fls_match_batch_begin")
+        arr_p, arr_n, stride, keep = _pack(scans)
+        Tc = _colmajor(Ts)
+        self._pending = (keep, arr_p, arr_n, Tc, len(scans))  # the asynchronous copies read these until match_batch_end
+        check(lib().fls_match_batch_begin(self._h, len(scans), arr_p, arr_n, stride, Tc.ctypes.data_as(C.c_void_p)), "fls_match_batch_begin")
 
     def match_batch_begin_device(self, d_ptrs, ns, Ts) -> None:
         """match_batch_begin with device-resident packed float4 scans."""
-        B = len(d_ptrs)
-        Tc = np.ascontiguousarray(np.transpose(np.asarray(Ts, np.float64), (0, 2, 1))).copy()
-        arr_p = (C.c_void_p * B)(*[int(p) for p in d_ptrs])
-        arr_n = (C.c_size_t * B)(*[int(n) for n in ns])
-        self._pending = ((), arr_p, arr_n, Tc, B)
-        check(lib().fls_match_batch_begin_device(self._h, B, arr_p, arr_n, Tc.ctypes.data_as(C.c_void_p)), "fls_match_batch_begin_device")
+        arr_p, arr_n = _pack_device(d_ptrs, ns)
+        Tc = _colmajor(Ts)
+        self._pending = ((), arr_p, arr_n, Tc, len(d_ptrs))
+        check(lib().fls_match_batch_begin_device(self._h, len(d_ptrs), arr_p, arr_n, Tc.ctypes.data_as(C.c_void_p)), "fls_match_batch_begin_device")
 
     def match_batch_end(self):
         keep, arr_p, arr_n, Tc, B = self._pending
-        conv = (C.c_int * B)()
-        st = (FlsMatchStats * B)()
+        conv, st = _batch_out(B)
         check(lib().fls_match_batch_end(self._h, Tc.ctypes.data_as(C.c_void_p), conv, st), "fls_match_batch_end")
         self._pending = None
-        self.last_batch_stats = list(st)
-        self.last_stats = st[0]
-        return np.array(conv[:], bool), np.transpose(Tc, (0, 2, 1)).copy()
+        return self._batch_result(Tc, conv, st)
 
     def match_batch_device(self, d_ptrs, ns, Ts):
         """Same with device-resident packed float4 scans: d_ptrs = list of device addresses, ns = point counts."""
-        B = len(d_ptrs)
-        Tc = np.ascontiguousarray(np.transpose(np.asarray(Ts, np.float64), (0, 2, 1))).copy()
-        conv = (C.c_int * B)()
-        st = (FlsMatchStats * B)()
-        arr_p = (C.c_void_p * B)(*[int(p) for p in d_ptrs])
-        arr_n = (C.c_size_t * B)(*[int(n) for n in ns])
-        check(lib().fls_match_batch_device(self._h, B, arr_p, arr_n, Tc.ctypes.data_as(C.c_void_p), conv, st), "fls_match_batch_device")
+        arr_p, arr_n = _pack_device(d_ptrs, ns)
+        Tc, (conv, st) = _colmajor(Ts), _batch_out(len(d_ptrs))
+        check(lib().fls_match_batch_device(self._h, len(d_ptrs), arr_p, arr_n, Tc.ctypes.data_as(C.c_void_p), conv, st), "fls_match_batch_device")
+        return self._batch_result(Tc, conv, st)
+
+    def _batch_result(self, Tc, conv, st):
         self.last_batch_stats = list(st)
         self.last_stats = st[0]
         return np.array(conv[:], bool), np.transpose(Tc, (0, 2, 1)).copy()
