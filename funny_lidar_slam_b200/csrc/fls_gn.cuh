@@ -33,6 +33,16 @@ struct GnLoopCtl {
 };
 static constexpr int kResultLen = 18;  // column-major 4x4 pose, converged, iterations
 
+// One scan of a batch launch (NDT, ICP, kd-tree point-to-plane): the grid is cut into one sub-grid per scan, scan s is served by
+// CTAs [cta0, cta0 + ncta) running its own persistent loop with its own arguments and control block
+template <class Args>
+struct __align__(16) GnBatchItem {
+    Args a;
+    GnLoopCtl ctl;
+    int cta0, ncta;
+    int pad[2];
+};
+
 void launch_gn_init(GnState* d_state, const double* T_colmajor, cudaStream_t st);
 
 #ifdef __CUDACC__
@@ -293,6 +303,26 @@ __device__ __forceinline__ bool gn_handover(double (&acc)[kNumAcc], const GnLoop
     }
     __syncthreads();
     return s_stop != 0;
+}
+
+// Prologue of a batch kernel: finds the item whose sub-grid holds this CTA and copies it into shared memory (`s_item`), so the
+// loop reads its arguments like kernel parameters.
+template <int BLOCK, class Args>
+__device__ __forceinline__ void gn_batch_item(const GnBatchItem<Args>* __restrict__ items, int n_scans, GnBatchItem<Args>& s_item) {
+    static_assert(sizeof(GnBatchItem<Args>) % 8 == 0, "copied in 8-byte words");
+    __shared__ int s_which;
+    if (threadIdx.x == 0) {
+        int w = 0;
+        while (w + 1 < n_scans && (int)blockIdx.x >= items[w + 1].cta0) ++w;
+        s_which = w;
+    }
+    __syncthreads();
+    {
+        const unsigned long long* src = reinterpret_cast<const unsigned long long*>(items + s_which);
+        unsigned long long* dst = reinterpret_cast<unsigned long long*>(&s_item);
+        for (int k = threadIdx.x; k < (int)(sizeof(GnBatchItem<Args>) / 8); k += BLOCK) dst[k] = src[k];
+    }
+    __syncthreads();
 }
 #endif
 

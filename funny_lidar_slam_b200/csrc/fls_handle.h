@@ -142,15 +142,18 @@ struct Handle {
 
     int add_cloud_ndt(const float4* d_cloud, size_t n);
     int match_ndt(const float4* d_src, size_t n, double* T, int* converged, fls_match_stats* st);
+    bool filter_batch(int n_scans, const float4* const* d_scans, const size_t* n_in, size_t* off, size_t* nf);  // ICP / NDT sources
     int match_ndt_batch(int n_scans, const float4* const* d_scans, const size_t* n, double* T, int* converged, fls_match_stats* st);
 
     int add_cloud_icp(const float4* d_cloud, size_t n);
     int match_icp(const float4* d_src, size_t n, double* T, int* converged, fls_match_stats* st);
+    int match_icp_batch(int n_scans, const float4* const* d_scans, const size_t* n, double* T, int* converged, fls_match_stats* st);
 
     // filter_mode 0: always VoxelGrid(leaf); 1: only once the window holds more than 5 clouds (loam_full_kdtree.h:91-99)
     int window_add(WindowMap& w, const float4* d_cloud, size_t n, size_t window, float leaf, int filter_mode, bool replace);
     int add_cloud_kd(const float4* d_planar, size_t n_planar, const float4* d_corner, size_t n_corner);
     int match_kd(const float4* d_planar, size_t n_planar, const float4* d_corner, size_t n_corner, double* T, int* converged, fls_match_stats* st);
+    int match_kd_batch(int n_scans, const float4* const* d_planar, const size_t* n, double* T, int* converged, fls_match_stats* st);  // FLS_P2PLANE_KNN
     bool need_add_cloud(const double* T, double* last_T, bool* have_last) const;
 
     int fitness(float max_range, float* score);

@@ -52,6 +52,7 @@ __device__ __forceinline__ bool grid_nn1(const IvoxView& g, float qx, float qy, 
 // sub, sub+kIcpLanes, ...; the winner is the lexicographic minimum of (d2, stencil position, point index) — the same
 // point the sequential scan above keeps (strict '<' in visit order).  All lanes of the group return the result.
 static constexpr int kIcpLanes = 8;
+static_assert(kIcpPerBlock * kIcpLanes == kIcpBlock, "fls_kernels.h sizes the sub-grids by kIcpPerBlock");
 __device__ __forceinline__ bool grid_nn1_coop(const IvoxView& g, int sub, unsigned group_mask, float qx, float qy, float qz, float& best_d,
                                               unsigned& best_j, unsigned& n_cand, unsigned& n_hits) {
     best_d = INFINITY;
@@ -94,9 +95,10 @@ __device__ __forceinline__ bool grid_nn1_coop(const IvoxView& g, int sub, unsign
     return best_j != 0xffffffffu;
 }
 
-// One persistent launch runs every Gauss-Newton iteration of a Match (gn_handover, fls_gn.cuh).
+// One persistent launch runs every Gauss-Newton iteration of a Match (gn_handover, fls_gn.cuh).  (cta, ncta): position of this
+// CTA in the (sub-)grid that serves the scan.
 template <int BLOCK>
-__global__ void __launch_bounds__(BLOCK) icp_gn_kernel(IcpArgs a, GnLoopCtl ctl) {
+__device__ __forceinline__ void icp_gn_loop(const IcpArgs& a, const GnLoopCtl& ctl, const int cta, const int ncta) {
     __shared__ double s_pose[12];
     __shared__ float s_posef[12];
     const int sub = threadIdx.x & (kIcpLanes - 1);
@@ -111,7 +113,7 @@ __global__ void __launch_bounds__(BLOCK) icp_gn_kernel(IcpArgs a, GnLoopCtl ctl)
 #pragma unroll
         for (int k = 0; k < kNumAcc; ++k) acc[k] = 0.0;
 
-        for (int i = blockIdx.x * kPerBlock + threadIdx.x / kIcpLanes; i < a.n; i += gridDim.x * kPerBlock) {
+        for (int i = cta * kPerBlock + threadIdx.x / kIcpLanes; i < a.n; i += ncta * kPerBlock) {
             const float4 sp = a.src[i];
             const float qx = xform_row_f(s_posef[0], s_posef[1], s_posef[2], s_posef[9], sp.x, sp.y, sp.z);
             const float qy = xform_row_f(s_posef[3], s_posef[4], s_posef[5], s_posef[10], sp.x, sp.y, sp.z);
@@ -151,8 +153,22 @@ __global__ void __launch_bounds__(BLOCK) icp_gn_kernel(IcpArgs a, GnLoopCtl ctl)
                 acc[kAccRes] += sqrt(e0 * e0 + e1 * e1 + e2 * e2);  // total_res += error.norm()  (:126)
             }
         }
-        if (gn_handover<BLOCK>(acc, ctl, it, s_pose)) break;
+        if (gn_handover<BLOCK>(acc, ctl, it, s_pose, cta, ncta)) break;
     }
+}
+
+template <int BLOCK>
+__global__ void __launch_bounds__(BLOCK) icp_gn_kernel(IcpArgs a, GnLoopCtl ctl) {
+    icp_gn_loop<BLOCK>(a, ctl, (int)blockIdx.x, (int)gridDim.x);
+}
+
+// A batch of independent scans against the same (static) map in ONE cooperative launch, a sub-grid and a loop per scan (as
+// ndt_gn_batch_kernel): the hand-over of one scan overlaps with the residual passes of the others.
+template <int BLOCK>
+__global__ void __launch_bounds__(BLOCK) icp_gn_batch_kernel(const IcpBatchItem* __restrict__ items, int n_scans) {
+    __shared__ IcpBatchItem s_item;
+    gn_batch_item<BLOCK>(items, n_scans, s_item);
+    icp_gn_loop<BLOCK>(s_item.a, s_item.ctl, (int)blockIdx.x - s_item.cta0, s_item.ncta);
 }
 
 // GetFitnessScore (icp_optimized.h:191-215 upstream): mean squared 1-NN distance over points with d2 <= max_range
@@ -203,8 +219,7 @@ int icp_grid_blocks(int n, int device) {
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, icp_gn_kernel<kIcpBlock>, kIcpBlock, 0);
         cap[device] = sms * (per_sm > 0 ? per_sm : 1);
     }
-    const int per_block = kIcpBlock / kIcpLanes;
-    const int need = (n + per_block - 1) / per_block;
+    const int need = (n + kIcpPerBlock - 1) / kIcpPerBlock;
     const int c = (device >= 0 && device < 64) ? cap[device] : 148;
     const int g = need < c ? need : c;
     return g > 0 ? g : 1;
@@ -214,6 +229,21 @@ void launch_icp_loop(const IcpArgs& a, const GnLoopCtl& ctl, int grid, cudaStrea
     GnLoopCtl c_ = ctl;
     void* params[] = {&a_, &c_};
     FLS_CUDA(cudaLaunchCooperativeKernel((const void*)icp_gn_kernel<kIcpBlock>, dim3(grid), dim3(kIcpBlock), params, 0, st));
+}
+
+int icp_max_grid(int device) {
+    static int cap[64] = {0};
+    if (device >= 0 && device < 64 && !cap[device]) {
+        int sms = 0, per_sm = 0;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, icp_gn_batch_kernel<kIcpBlock>, kIcpBlock, 0);
+        cap[device] = sms * (per_sm > 0 ? per_sm : 1);
+    }
+    return (device >= 0 && device < 64) ? cap[device] : 148;
+}
+void launch_icp_batch(const IcpBatchItem* d_items, int n_scans, int grid, cudaStream_t st) {
+    void* params[] = {&d_items, &n_scans};
+    FLS_CUDA(cudaLaunchCooperativeKernel((const void*)icp_gn_batch_kernel<kIcpBlock>, dim3(grid), dim3(kIcpBlock), params, 0, st));
 }
 
 void launch_fitness(const IvoxView& g, const float4* d_src, int n, const double* T, float max_range, double* d_out2, cudaStream_t st) {

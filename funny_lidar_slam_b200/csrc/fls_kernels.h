@@ -1,4 +1,4 @@
-// fls_kernels.h — launch interfaces of the residual kernels (K1 p2plane/iVox, K2 NDT, K3 ICP) and GetFitnessScore.
+// fls_kernels.h — launch interfaces of the residual kernels (K1 p2plane/iVox, K2 NDT, K3 ICP, K5 kd-tree LOAM) and GetFitnessScore.
 #pragma once
 #include "fls_common.cuh"
 #include "fls_gn.cuh"
@@ -74,12 +74,7 @@ struct NdtArgs {
 int ndt_grid(int n, int device);  // co-resident grid of the persistent kernel
 void launch_ndt_loop(const NdtArgs& a, const GnLoopCtl& ctl, int grid, cudaStream_t st);
 // batch of scans in one launch: scan s is served by CTAs [cta0, cta0 + ncta) of the grid (its own persistent loop)
-struct __align__(16) NdtBatchItem {
-    NdtArgs a;
-    GnLoopCtl ctl;
-    int cta0, ncta;
-    int pad[2];
-};
+using NdtBatchItem = GnBatchItem<NdtArgs>;
 int ndt_max_grid(int device);  // co-resident CTAs of the batch kernel
 void launch_ndt_batch(const NdtBatchItem* d_items, int n_scans, int grid, cudaStream_t st);
 
@@ -92,6 +87,10 @@ struct IcpArgs {
 };
 int icp_grid_blocks(int n, int device);
 void launch_icp_loop(const IcpArgs& a, const GnLoopCtl& ctl, int grid, cudaStream_t st);
+static constexpr int kIcpPerBlock = kIcpBlock / 8;  // queries per CTA (8 lanes share one)
+using IcpBatchItem = GnBatchItem<IcpArgs>;
+int icp_max_grid(int device);  // co-resident CTAs of the batch kernel
+void launch_icp_batch(const IcpBatchItem* d_items, int n_scans, int grid, cudaStream_t st);
 
 // K5 — kd-tree LOAM plug-ins (LoamPointToPlaneKdtree, LoamFull): exact unbounded 5-NN over a uniform grid
 struct LoamGrid {
@@ -117,6 +116,11 @@ struct LoamArgs {
 };
 int loam_grid_blocks(int n, int device);
 void launch_loam_loop(const LoamArgs& a, const GnLoopCtl& ctl, int grid, cudaStream_t st);
+static constexpr int kLoamPerBlock = kLoamBlock / 8;  // queries per CTA (8 lanes share one)
+using LoamBatchItem = GnBatchItem<LoamArgs>;
+int loam_max_grid(int device);  // co-resident CTAs of the batch kernel
+// clears the flags of all `n_flags` points of the batch (once per Match [quirk 1]), then runs the batch in one launch
+void launch_loam_batch(const LoamBatchItem* d_items, int n_scans, int grid, unsigned char* flags, int n_flags, cudaStream_t st);
 
 // d_out2[0] = sum of squared NN distances <= max_range, d_out2[1] = how many; T column-major (cast to float inside)
 void launch_fitness(const IvoxView& g, const float4* d_src, int n, const double* T_colmajor, float max_range, double* d_out2, cudaStream_t st);

@@ -40,6 +40,7 @@ __device__ __forceinline__ void scan_cell(const LoamGrid& g, int cx, int cy, int
 // kLoamLanes lanes share one query: lane `sub` visits every kLoamLanes-th cell, keeps a PRIVATE top-5 (the private lists
 // of a group are disjoint), and the group's answer is their butterfly merge.
 static constexpr int kLoamLanes = 8;
+static_assert(kLoamPerBlock * kLoamLanes == kLoamBlock, "fls_kernels.h sizes the sub-grids by kLoamPerBlock");
 
 __device__ __forceinline__ void merge_group(Top5& m, unsigned group_mask) {
 #pragma unroll
@@ -151,8 +152,10 @@ __device__ __forceinline__ bool corner_term(const float4* __restrict__ P, const 
     return true;
 }
 
+// (cta, ncta): position of this CTA in the (sub-)grid that serves the scan.  `a` by value: as a reference it costs the single-scan
+// kernel 32 more bytes of stack frame (grid_knn5 takes the address of a map view).
 template <int BLOCK>
-__global__ void __launch_bounds__(BLOCK) loam_gn_kernel(LoamArgs a, GnLoopCtl ctl) {
+__device__ __forceinline__ void loam_gn_loop(const LoamArgs a, const GnLoopCtl& ctl, const int cta, const int ncta) {
     __shared__ double s_pose[12];
     const int n_total = a.n_corner + a.n_planar;
     const int sub = threadIdx.x & (kLoamLanes - 1);
@@ -164,7 +167,7 @@ __global__ void __launch_bounds__(BLOCK) loam_gn_kernel(LoamArgs a, GnLoopCtl ct
         double acc[kNumAcc];
 #pragma unroll
         for (int k = 0; k < kNumAcc; ++k) acc[k] = 0.0;
-        for (int i = blockIdx.x * kPerBlock + threadIdx.x / kLoamLanes; i < n_total; i += gridDim.x * kPerBlock) {
+        for (int i = cta * kPerBlock + threadIdx.x / kLoamLanes; i < n_total; i += ncta * kPerBlock) {
             const bool is_corner = i < a.n_corner;
             const float4 sp = is_corner ? a.corner[i] : a.planar[i - a.n_corner];
             // pcl::transformPoint with the double transform, stored back as fp32 (:219-220, :284-285, kdtree :211-212)
@@ -209,8 +212,22 @@ __global__ void __launch_bounds__(BLOCK) loam_gn_kernel(LoamArgs a, GnLoopCtl ct
                 else acc[kAccValid] += 1.0;           // number_valid_planar_ (the < 50 failure test)
             }
         }
-        if (gn_handover<BLOCK>(acc, ctl, it, s_pose)) break;
+        if (gn_handover<BLOCK>(acc, ctl, it, s_pose, cta, ncta)) break;
     }
+}
+
+template <int BLOCK>
+__global__ void __launch_bounds__(BLOCK) loam_gn_kernel(LoamArgs a, GnLoopCtl ctl) {
+    loam_gn_loop<BLOCK>(a, ctl, (int)blockIdx.x, (int)gridDim.x);
+}
+
+// A batch of independent LoamPointToPlaneKdtree scans (planar only) against the same (static) map in ONE cooperative launch, a
+// sub-grid and a loop per scan (as ndt_gn_batch_kernel); every scan owns its slice of the records and flags.
+template <int BLOCK>
+__global__ void __launch_bounds__(BLOCK) loam_gn_batch_kernel(const LoamBatchItem* __restrict__ items, int n_scans) {
+    __shared__ LoamBatchItem s_item;
+    gn_batch_item<BLOCK>(items, n_scans, s_item);
+    loam_gn_loop<BLOCK>(s_item.a, s_item.ctl, (int)blockIdx.x - s_item.cta0, s_item.ncta);
 }
 
 __global__ void loam_clear_flags_kernel(unsigned char* flags, int n) {
@@ -228,8 +245,7 @@ int loam_grid_blocks(int n, int device) {
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, loam_gn_kernel<kLoamBlock>, kLoamBlock, 0);
         cap[device] = sms * (per_sm > 0 ? per_sm : 1);
     }
-    const int per_block = kLoamBlock / kLoamLanes;
-    const int need = (n + per_block - 1) / per_block;
+    const int need = (n + kLoamPerBlock - 1) / kLoamPerBlock;
     const int c = (device >= 0 && device < 64) ? cap[device] : 148;
     const int g = need < c ? need : c;
     return g > 0 ? g : 1;
@@ -242,6 +258,23 @@ void launch_loam_loop(const LoamArgs& a, const GnLoopCtl& ctl, int grid, cudaStr
     if (n > 0) loam_clear_flags_kernel<<<(n + 255) / 256, 256, 0, st>>>(a.flags, n);
     void* params[] = {&a_, &c_};
     FLS_CUDA(cudaLaunchCooperativeKernel((const void*)loam_gn_kernel<kLoamBlock>, dim3(grid), dim3(kLoamBlock), params, 0, st));
+}
+
+int loam_max_grid(int device) {
+    static int cap[64] = {0};
+    if (device >= 0 && device < 64 && !cap[device]) {
+        int sms = 0, per_sm = 0;
+        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, loam_gn_batch_kernel<kLoamBlock>, kLoamBlock, 0);
+        cap[device] = sms * (per_sm > 0 ? per_sm : 1);
+    }
+    return (device >= 0 && device < 64) ? cap[device] : 148;
+}
+
+void launch_loam_batch(const LoamBatchItem* d_items, int n_scans, int grid, unsigned char* flags, int n_flags, cudaStream_t st) {
+    if (n_flags > 0) loam_clear_flags_kernel<<<(n_flags + 255) / 256, 256, 0, st>>>(flags, n_flags);
+    void* params[] = {&d_items, &n_scans};
+    FLS_CUDA(cudaLaunchCooperativeKernel((const void*)loam_gn_batch_kernel<kLoamBlock>, dim3(grid), dim3(kLoamBlock), params, 0, st));
 }
 
 }  // namespace fls

@@ -394,19 +394,7 @@ __global__ void __launch_bounds__(BLOCK) ndt_gn_kernel(NdtArgs a, GnLoopCtl ctl)
 template <int BLOCK>
 __global__ void __launch_bounds__(BLOCK) ndt_gn_batch_kernel(const NdtBatchItem* __restrict__ items, int n_scans) {
     __shared__ NdtBatchItem s_item;
-    __shared__ int s_which;
-    if (threadIdx.x == 0) {
-        int w = 0;
-        while (w + 1 < n_scans && (int)blockIdx.x >= items[w + 1].cta0) ++w;
-        s_which = w;
-    }
-    __syncthreads();
-    {
-        const unsigned long long* src = reinterpret_cast<const unsigned long long*>(items + s_which);
-        unsigned long long* dst = reinterpret_cast<unsigned long long*>(&s_item);
-        for (int k = threadIdx.x; k < (int)(sizeof(NdtBatchItem) / 8); k += BLOCK) dst[k] = src[k];
-    }
-    __syncthreads();
+    gn_batch_item<BLOCK>(items, n_scans, s_item);
     ndt_gn_loop<BLOCK>(s_item.a, s_item.ctl, (int)blockIdx.x - s_item.cta0, s_item.ncta);
 }
 

@@ -108,10 +108,12 @@ class Registration:
         check(rc, "fls_fitness")
         return float(out.value)
 
-    # -- batched Match (throughput entry; LoamPointToPlaneIVOX in localization mode) -----------------------------
+    # -- batched Match (throughput entry: LoamPointToPlaneIVOX, IncrementalNDT, IcpOptimized, LoamPointToPlaneKdtree) ------
     def match_batch(self, scans, Ts):
-        """scans: list of (n,4)/(n,8) host clouds; Ts: (B,4,4) float64 initial poses.  Returns (converged[B], T[B,4,4]);
-        self.last_batch_stats holds the per-scan fls_match_stats (call-level timings on element 0)."""
+        """scans: list of (n,4)/(n,8) host clouds — the planar clouds for the LOAM point-to-plane plug-ins (iVox and kd-tree), the
+        ordered clouds for NDT and ICP; Ts: (B,4,4) float64 initial poses.  Returns (converged[B], T[B,4,4]);
+        self.last_batch_stats holds the per-scan fls_match_stats (call-level timings on element 0).  More than one scan needs
+        localization mode; LoamFull has no batch entry.  GetFitnessScore afterwards scores scan 0 at its final pose."""
         arr_p, arr_n, stride, keep = _pack(scans)
         Tc, (conv, st) = _colmajor(Ts), _batch_out(len(scans))
         check(lib().fls_match_batch(self._h, len(scans), arr_p, arr_n, stride, Tc.ctypes.data_as(C.c_void_p), conv, st), "fls_match_batch")
@@ -140,7 +142,8 @@ class Registration:
         return self._batch_result(Tc, conv, st)
 
     def match_batch_device(self, d_ptrs, ns, Ts):
-        """Same with device-resident packed float4 scans: d_ptrs = list of device addresses, ns = point counts."""
+        """Same with device-resident packed float4 scans: d_ptrs = list of device addresses, ns = point counts.  Same plug-ins and
+        clouds as match_batch."""
         arr_p, arr_n = _pack_device(d_ptrs, ns)
         Tc, (conv, st) = _colmajor(Ts), _batch_out(len(d_ptrs))
         check(lib().fls_match_batch_device(self._h, len(d_ptrs), arr_p, arr_n, Tc.ctypes.data_as(C.c_void_p), conv, st), "fls_match_batch_device")

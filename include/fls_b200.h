@@ -175,14 +175,18 @@ int fls_match(fls_handle* h, const void* ordered, size_t n_ordered, const void* 
  * meaningful only when the call returns FLS_OK. */
 int fls_match_device(fls_handle* h, const void* d_points, size_t n, double T_colmajor[16], int* converged, fls_match_stats* stats);
 
-/* GetFitnessScore(max_range): FLT_MAX when unsupported / no inliers, as upstream. */
+/* GetFitnessScore(max_range): FLT_MAX when unsupported / no inliers, as upstream.  After a batch (fls_match_batch*) it scores scan 0
+ * of the batch at its final pose, with the same cloud its single Match would leave. */
 int fls_fitness(fls_handle* h, float max_range, float* score);
 
 /* Batched Match for throughput (the benchmark entry SURVEY.md §8b names): `n_scans` (<= 64) independent scans, each with its
  * own in-out pose T[s*16 .. s*16+15], converged[s] and stats[s], matched against the same map in ONE persistent launch.
- * Implemented for FLS_P2PLANE_IVOX (one persistent work-queue kernel for the batch) and FLS_NDT (one cooperative launch, a
- * sub-grid and a Gauss-Newton loop per scan); more than one scan requires localization_mode (Match must not modify the map).
- * For the LOAM-iVox plug-in the entry reads the planar clouds, for NDT the ordered clouds of the scans.
+ * Implemented for FLS_P2PLANE_IVOX (one persistent work-queue kernel for the batch), and for FLS_NDT, FLS_ICP_P2P and
+ * FLS_P2PLANE_KNN (one cooperative launch, a sub-grid and a Gauss-Newton loop per scan); FLS_LOAM_FULL returns
+ * FLS_ERR_UNSUPPORTED (its Match inserts key frames even in localization mode, and it needs corner clouds).  More than one scan
+ * requires localization_mode (Match must not modify the map); a batch of one is exactly fls_match, in either mode.
+ * The entry reads the planar clouds for FLS_P2PLANE_IVOX and FLS_P2PLANE_KNN, the ordered clouds for FLS_NDT and FLS_ICP_P2P.
+ * An FLS_ICP_P2P batch with a scan of <= 10 points is refused as a whole (FLS_ERR_TOO_FEW_POINTS) before anything runs.
  * Call-level figures (gpu_ms, gpu_launches, byte counts, kernel_ms) are reported in stats[0]; per-scan fields everywhere.
  * Results are identical to n_scans separate fls_match calls.  The _device variant takes device pointers to packed float4 scans. */
 int fls_match_batch(fls_handle* h, int n_scans, const void* const* planar, const size_t* n, size_t stride_bytes, double* T_colmajor,
